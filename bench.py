@@ -5,7 +5,7 @@ One "step" = one frame of the BASELINE config-2 pipeline: GridSample(voxel 0.3) 
 ICPFrameToModel (kd-tree local map of 20 frames, point-to-plane Gauss-Newton, geman_mcclure
 sigma 0.3, <= 10 alignments, constant-velocity initialisation), on a seeded synthetic stream.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-extra] [--no-cpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-extra] [--no-cpu] [--dump-outputs DIR]
 
 * `value`  : frames/s with every raw scan already resident in HBM; one C-ABI call per frame
              (pls_process_frame_grid_sample) on device pointers; ONE CUDA-event bracket on the library's
@@ -26,7 +26,11 @@ sigma 0.3, <= 10 alignments, constant-velocity initialisation), on a seeded synt
              sharded over the ranks.
 * config.sharded_vs_single (N > 1): poses of a forced-sharded run against rank 0's private single-GPU context.
 * cpu_baseline / --impl reference: the CPU oracle port of the reference path (oracle/) on the host
-             cores, on a bounded sample of the same stream.
+             cores, on a bounded sample of the same stream (--impl reference: at most 24 warm-up frames, then K timed frames).
+* --dump-outputs DIR: after the timed passes, what the timed call returned for the last timed frame, as DIR/<name>.npy:
+             odometry_pose [4,4] float32, odometry_params [6] float32, frame_info [12] float64 (pls_process_frame's
+             out_info); the pass whose time is reported.  --impl reference writes odometry_pose [4,4] float64 alone.
+             The scans are seeded, so the same arguments give the same inputs on every run and build.
 """
 import argparse
 import ctypes as C
@@ -132,6 +136,12 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons)}
 
 
+def dump_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
+
 def make_scans(n_frames, h=H, w=W):
     from pylidar_slam_b200 import synthetic as syn
     return [syn.scan(k, h, w) for k in range(n_frames)]
@@ -224,12 +234,14 @@ def reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # bounded sample: the map needs ~20 frames to reach steady state; cap the CPU work at ~55 frames
+    # the map needs ~20 frames to reach steady state; more warm-up only costs CPU time
     warmup = min(args.warmup, 24)
-    steps = min(args.steps, 30)
+    steps = args.steps
     scans = make_scans(warmup + steps)
     t0 = time.perf_counter()
-    fps, times, cal, _ = run_cpu_port(scans, warmup, steps, calibrate=True)
+    fps, times, cal, last_pose = run_cpu_port(scans, warmup, steps, calibrate=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"odometry_pose": np.asarray(last_pose, np.float64)})
     line = {
         "impl": "reference", "metric": "icp_odometry_frames_per_sec", "value": fps, "unit": "frames/s",
         "n_gpus": args.gpus, "steps": steps, "warmup": warmup, "ms_per_step": 1e3 * float(np.mean(times)),
@@ -377,7 +389,8 @@ def b200_arm(args):
         prof = ctx.profile(profile_slot) if profile_slot is not None else None
         stats = {"samples": int(info[4]), "queries": int(info[2]), "map_points": int(info[3]), "iters_mean": float(np.mean(iters)),
                  "iters_total": int(np.sum(iters)), "frames_sharded": sharded}
-        return total_ms, launches, prof, stats
+        last = {"odometry_pose": pose.copy(), "odometry_params": params.copy(), "frame_info": info.copy()}
+        return total_ms, launches, prof, stats, last
 
     clocks = ClockSampler(local_rank, enabled=(rank == 0))
     clocks.start()
@@ -385,7 +398,9 @@ def b200_arm(args):
     # with the driver's --steps 20 one bracket is a 10 ms sample; every pass is listed in config.repeats
     value_passes = [device_pass() for _ in range(1 if args.quick else REPEATS)]
     clock_info = clocks.stop()
-    ms_dev, launches, _, stats = sorted(value_passes, key=lambda r: r[0])[len(value_passes) // 2]
+    ms_dev, launches, _, stats, last = sorted(value_passes, key=lambda r: r[0])[len(value_passes) // 2]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     if args.quick:
         (ms_dev,) = max_over_ranks(ms_dev)
         if world > 1:
@@ -394,11 +409,11 @@ def b200_arm(args):
             print(json.dumps({"quick": True, "n_gpus": world, "comm": comm_used[0] if world > 1 else None,
                               "ms_per_step": ms_dev / K_, "gpu_launches": launches, **stats}))
         return
-    ms_dev_flushed, _, _, _ = device_pass(flush_each_step=True)
+    ms_dev_flushed, _, _, _, _ = device_pass(flush_each_step=True)
     # roofline passes: same frames with CUDA events around one kernel family inside the library
-    _, _, prof_nn, stats_nn = device_pass(profile_slot=0)
-    _, _, prof_idx, _ = device_pass(profile_slot=3)
-    _, _, prof_gs, _ = device_pass(profile_slot=4)
+    _, _, prof_nn, stats_nn, _ = device_pass(profile_slot=0)
+    _, _, prof_idx, _, _ = device_pass(profile_slot=3)
+    _, _, prof_gs, _, _ = device_pass(profile_slot=4)
 
     # ---------------- e2e: reference-shaped Python API from pinned host buffers
     pinned = [torch.from_numpy(s).pin_memory() for s in scans]
@@ -684,7 +699,11 @@ def main():
     ap.add_argument("--quick", action="store_true", help="device-resident pass only (for ncu captures)")
     ap.add_argument("--comm", default="p2p", choices=["p2p", "nccl"],
                     help="N>1 exchange: one-shot NVLink peer-to-peer all-reduce fused into the solve kernel, or NCCL")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed path's outputs of its last timed frame to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -16,7 +16,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GENERATORS = ["make_golden_misc", "make_golden_gn", "make_golden_io", "make_golden_chain", "make_golden_loss",
-              "make_golden_next", "make_golden"]
+              "make_golden_next", "make_golden", "make_golden_dropin"]
 
 
 def same(x, y):

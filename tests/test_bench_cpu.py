@@ -42,8 +42,9 @@ def test_thread_calibration_does_not_disturb_the_stream(monkeypatch):
         torch.set_num_threads(before)
 
 
-def test_reference_arm_prints_one_contract_line():
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "3"],
+def test_reference_arm_prints_one_contract_line(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "3",
+                          "--dump-outputs", str(tmp_path)],
                          capture_output=True, text=True, timeout=600, cwd=ROOT, env={**os.environ, "RANK": "0"})
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
@@ -57,6 +58,9 @@ def test_reference_arm_prints_one_contract_line():
     assert cb["kind"] == "port" and cb["value"] == d["value"] and cb["cores"] == os.cpu_count() and cb["torch_threads"] >= 1
     assert cb["kd_workers"] in (-1, 1, 8, 32) and "calibrated" in cb["sample"]
     assert d["config"]["workload"].startswith("cfg2") and d["config"]["height"] == 64 and d["config"]["width"] == 2048
+    assert os.listdir(tmp_path) == ["odometry_pose.npy"]
+    pose = np.load(tmp_path / "odometry_pose.npy")
+    assert pose.shape == (4, 4) and pose.dtype == np.float64 and np.isfinite(pose).all()
 
 
 def test_reference_arm_is_silent_on_other_ranks():
@@ -168,7 +172,7 @@ def _bench_fakes(monkeypatch):
     return BenchFakeContext
 
 
-def test_b200_arm_assembles_the_contract_line_dry_run(monkeypatch, capsys):
+def test_b200_arm_assembles_the_contract_line_dry_run(monkeypatch, capsys, tmp_path):
     import argparse
     import bench
     from pylidar_slam_b200 import _lib
@@ -186,11 +190,18 @@ def test_b200_arm_assembles_the_contract_line_dry_run(monkeypatch, capsys):
     def failing_extras(*a, **k):                # an extra workload that dies must not take the headline line with it
         raise RuntimeError("extra workload failed (dry run)")
     monkeypatch.setattr(bench, "extra_workloads", failing_extras)
-    args = argparse.Namespace(gpus=1, steps=4, warmup=3, impl="b200", no_cpu=False, no_extra=False, quick=False, comm="p2p")
+    args = argparse.Namespace(gpus=1, steps=4, warmup=3, impl="b200", no_cpu=False, no_extra=False, quick=False, comm="p2p",
+                              dump_outputs=str(tmp_path / "out"))
     bench.b200_arm(args)
     lines = [l for l in capsys.readouterr().out.splitlines() if l.startswith("{")]
     assert len(lines) == 1
     d = json.loads(lines[0])
+    # --dump-outputs: the last timed frame's outputs of the timed call (frame 1 + W + K - 1 of the seeded stream)
+    dumped = {f: np.load(tmp_path / "out" / f) for f in sorted(os.listdir(tmp_path / "out"))}
+    assert {f: (a.shape, a.dtype) for f, a in dumped.items()} == {
+        "frame_info.npy": ((12,), np.float64), "odometry_params.npy": ((6,), np.float32), "odometry_pose.npy": ((4, 4), np.float32)}
+    assert np.isfinite(dumped["odometry_pose.npy"]).all() and not np.array_equal(dumped["odometry_pose.npy"], np.eye(4))
+    assert dumped["frame_info.npy"][0] >= 1 and dumped["frame_info.npy"][4] == d["config"]["samples"]
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
                 "vs_baseline", "dtype", "data", "config", "e2e", "gpu_launches", "clocks", "roofline", "kernels"):
         assert key in d, key
@@ -253,7 +264,8 @@ def _two_rank_worker(rank, world, port, out):
     bench.make_scans = lambda n, h=32, w=512: [syn.scan(k, h, w) for k in range(n)]
     bench.extra_workloads = lambda *a, **k: {"stub": True}
     torch.set_num_threads(1)
-    args = argparse.Namespace(gpus=world, steps=3, warmup=3, impl="b200", no_cpu=False, no_extra=False, quick=False, comm="p2p")
+    args = argparse.Namespace(gpus=world, steps=3, warmup=3, impl="b200", no_cpu=False, no_extra=False, quick=False, comm="p2p",
+                              dump_outputs=None)
     buf = io.StringIO()
     with contextlib.redirect_stdout(buf):
         bench.b200_arm(args)
